@@ -23,6 +23,8 @@ A "step" = forward + backward + (NCCL all-reduce) + clip + AdamW on one batch of
             real (unpadded) tokens/s, `packed_steps`, `length_groups_per_step`.  DTX_VARLEN_SPLIT=0 / DTX_VARLEN_PACK=0: one pass
             at the padded shape / length groups, for A/B runs.
 Other configs (not the headline metric): mistral7b_qlora (BASELINE configs[2]), 13b_full (configs[3], 8 GPUs), small_full, tiny.
+`--dump-outputs DIR`: loss, grad-norm, lr of the last timed device-resident step and the trainable parameters after it, as .npy
+            (seeded inputs and weights: the same arguments give the same inputs, so two builds compare array for array).
 """
 from __future__ import annotations
 
@@ -287,6 +289,28 @@ def varlen_lengths(step: int, rank: int, batch: int, seq_len: int) -> np.ndarray
     return np.clip(np.exp(rng.normal(np.log(seq_len / 4.0), 0.6, size=batch)), 16, seq_len).astype(np.int32)
 
 
+DUMP_BYTES = 64 << 20  # what --dump-outputs may write in all
+
+
+def dump_outputs(tr, out_dir: str, last_step, full: bool) -> None:
+    """--dump-outputs: what the last device-resident timed step handed back - loss, grad-norm and learning rate - and the
+    trainable parameters it left behind, one DIR/<checkpoint name>.npy each: the PEFT adapters (fp32) or, for a full fine-tune,
+    the bf16 weights widened to fp32.  When the parameters exceed the budget, every tensor is cut to the same fraction of its
+    elements at positions drawn from a fixed per-tensor seed (flattened, in index order)."""
+    os.makedirs(out_dir, exist_ok=True)
+    loss, gnorm, lr, _ = last_step
+    arrays = {"loss": np.float32([loss]), "grad_norm": np.float32([gnorm]), "lr": np.float32([lr])}
+    params = tr.export_weights() if full else tr.export_adapter()
+    frac = min(1.0, (DUMP_BYTES - (1 << 20)) / (4.0 * sum(a.size for a in params.values())))  # 1 MB left for headers, scalars
+    for i, (name, a) in enumerate(params.items()):
+        if frac < 1.0:
+            idx = np.sort(np.random.default_rng(i).choice(a.size, size=max(1, int(a.size * frac)), replace=False))
+            a = a.reshape(-1)[idx]
+        arrays[name] = (a.astype(np.uint32) << 16).view(np.float32) if full else a
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_native(args, rank: int, local_rank: int, world: int):
     import torch  # device memory for the resident batches, gloo rendezvous and the clock; no torch compute
     from datatunerx_b200 import lib as L
@@ -367,9 +391,9 @@ def run_native(args, rank: int, local_rank: int, world: int):
         a, b, l = (dev if on_device else pinned)[i % n_batches]
         cur = lens_host[i % n_batches][1]
         return tr.step_ptr(a.data_ptr(), b.data_ptr(), on_device=on_device, seq_lens_ptr=l.data_ptr() if varlen else 0,
-                           seq_len_batch=cur)[0]
+                           seq_len_batch=cur)
 
-    losses = [run(i, True) for i in range(args.warmup)]
+    losses = [run(i, True)[0] for i in range(args.warmup)]
 
     sampler = ClockSampler(local_rank)
     sampler.start()
@@ -382,7 +406,8 @@ def run_native(args, rank: int, local_rank: int, world: int):
     dev_ms, segs, groups = [], [], []
     real_tokens = padded_tokens = 0
     for i in range(args.steps):
-        losses.append(run(i, True))
+        last = run(i, True)
+        losses.append(last[0])
         groups.append(tr.last_step_groups)
         dev_ms.append(tr.last_step_ms)
         segs.append(tr.last_step_timings)
@@ -393,11 +418,13 @@ def run_native(args, rank: int, local_rank: int, world: int):
     e1 = meter.read_j()
     dt = rv.max_over_ranks(dt_local)
     launches = tr.launch_count - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(tr, args.dump_outputs, last, full)
     # ---- timed region 2: end to end through the host API (pinned host batches in, loss out) ----
     barrier()
     t0 = time.perf_counter()
     for i in range(args.steps):
-        losses.append(run(i, False))
+        losses.append(run(i, False)[0])
     barrier()
     dt_e2e = rv.max_over_ranks(time.perf_counter() - t0)
     clocks = sampler.stop()
@@ -488,7 +515,13 @@ def main():
     ap.add_argument("--impl", default="native", choices=["native", "reference"])
     ap.add_argument("--config", default="7b", choices=["7b", "7b_varlen", "mistral7b_qlora", "13b_full", "small_full", "tiny"])
     ap.add_argument("--no-cpu-baseline", dest="cpu_baseline", action="store_false")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last device-resident step "
+                    "returned and the trainable parameters it left (rank 0) as DIR/<name>.npy, float32, <= 64 MB in all")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs needs --impl native")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
