@@ -123,6 +123,11 @@ int32_t dtx_swiglu_bwd(const void* dact, const void* gu, void* dgu, int32_t M, i
 int32_t dtx_lora_dropout_fwd(const void* h, void* hd, int32_t M, int32_t d, int32_t nt, float p, uint64_t key, void* stream) {
   return rc(lora_dropout_fwd(static_cast<const bf16*>(h), static_cast<bf16*>(hd), M, d, nt, p, key, S(stream)));
 }
+int32_t dtx_swiglu_bwd_lora_dropout(const void* dact, const void* g, const void* gu, void* dgu, int32_t M, int32_t F,
+                                    int32_t interleaved, float p, uint64_t key, void* stream) {
+  return rc(swiglu_bwd_lora_dropout(static_cast<const bf16*>(dact), static_cast<const bf16*>(g), static_cast<const bf16*>(gu),
+                                    static_cast<bf16*>(dgu), M, F, interleaved, p, key, S(stream)));
+}
 int32_t dtx_lora_dropout_bwd_add(void* dh, const void* g, int32_t M, int32_t d, int32_t nt, float p, uint64_t key, void* stream) {
   return rc(lora_dropout_bwd_add(static_cast<bf16*>(dh), static_cast<const bf16*>(g), M, d, nt, p, key, S(stream)));
 }

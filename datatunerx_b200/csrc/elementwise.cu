@@ -244,8 +244,12 @@ __global__ void swiglu_fwd_kernel(const bf16* __restrict__ gu, bf16* __restrict_
     reinterpret_cast<uint4*>(act + m * static_cast<long long>(F))[v] = f32_to_bf16x8(fg);
   }
 }
+__device__ __forceinline__ bool drop_keep(uint64_t key, int target, long long idx, uint32_t thresh);
+// glora (optional): LoRA dropout on down_proj's input - d(act) = dact + mask o glora / (1 - p), the mask regenerated (target 0
+// of `key`, element m*F + f), so that the masked LoRA-branch gradient joins the SwiGLU backward without another pass over HBM
 __global__ void swiglu_bwd_kernel(const bf16* __restrict__ dact, const bf16* __restrict__ gu, bf16* __restrict__ dgu,
-                                  int M, int F, int il) {
+                                  int M, int F, int il, const bf16* __restrict__ glora = nullptr, uint32_t thresh = 0,
+                                  float inv_keep = 1.f, uint64_t key = 0) {
   const int vecF = F >> 3;
   const long long total = static_cast<long long>(M) * vecF;
   for (long long t = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; t < total;
@@ -259,6 +263,13 @@ __global__ void swiglu_bwd_kernel(const bf16* __restrict__ dact, const bf16* __r
     bf16x8_to_f32(ldg_stream(reinterpret_cast<const uint4*>(gu + m * 2LL * F + gpos)), fg);
     bf16x8_to_f32(ldg_stream(reinterpret_cast<const uint4*>(gu + m * 2LL * F + upos)), fu);
     bf16x8_to_f32(ldg_stream(reinterpret_cast<const uint4*>(dact + m * static_cast<long long>(F)) + v), fd);
+    if (glora) {
+      float fl[8];
+      bf16x8_to_f32(ldg_stream(reinterpret_cast<const uint4*>(glora + m * static_cast<long long>(F)) + v), fl);
+#pragma unroll
+      for (int j = 0; j < 8; ++j)
+        if (drop_keep(key, 0, m * F + f + j, thresh)) fd[j] += fl[j] * inv_keep;
+    }
 #pragma unroll
     for (int j = 0; j < 8; ++j) {
       const float s = 1.f / (1.f + __expf(-fg[j]));
@@ -985,6 +996,13 @@ cudaError_t lora_dropout_bwd_add(bf16* dh, const bf16* g, int M, int d, int nt, 
   if (d % 8) return cudaErrorInvalidValue;
   lora_dropout_bwd_kernel<<<grid_for(static_cast<long long>(M) * (d / 8), 256), 256, 0, s>>>(dh, g, M, d, nt, drop_thresh(p),
                                                                                           1.0f / (1.0f - p), key);
+  return cudaGetLastError();
+}
+cudaError_t swiglu_bwd_lora_dropout(const bf16* dact, const bf16* g, const bf16* gu, bf16* dgu, int M, int F, int interleaved, float p,
+                                    uint64_t key, cudaStream_t s) {
+  if (!g || F % 8 || (interleaved && F % 128)) return cudaErrorInvalidValue;
+  swiglu_bwd_kernel<<<grid_for(static_cast<long long>(M) * (F / 8), 256), 256, 0, s>>>(dact, gu, dgu, M, F, interleaved, g, drop_thresh(p),
+                                                                                    1.0f / (1.0f - p), key);
   return cudaGetLastError();
 }
 

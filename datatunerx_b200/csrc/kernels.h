@@ -163,6 +163,10 @@ cudaError_t adamw_step(const AdamWArgs& a, cudaStream_t s);
 // dh[M, d] += sum_t mask_t o g[:, t*d:(t+1)*d] / (1-p)
 cudaError_t lora_dropout_fwd(const bf16* h, bf16* hd, int M, int d, int nt, float p, uint64_t key, cudaStream_t s);
 cudaError_t lora_dropout_bwd_add(bf16* dh, const bf16* g, int M, int d, int nt, float p, uint64_t key, cudaStream_t s);
+// LoRA dropout on down_proj's input, backward: dgu[M,2F] = SwiGLU backward of d(act) = dact + mask o g / (1-p) (g [M,F] = the
+// LoRA branch's input gradient; mask = target 0 of `key`, element m*F + f, as lora_dropout_fwd with d = F) in one pass
+cudaError_t swiglu_bwd_lora_dropout(const bf16* dact, const bf16* g, const bf16* gu, bf16* dgu, int M, int F, int interleaved, float p,
+                                    uint64_t key, cudaStream_t s);
 // fp32 -> bf16 with scale, strided 2-D (used to refresh the bf16 LoRA shadows)
 cudaError_t cast_f32_to_bf16_2d(const float* src, int64_t lds, bf16* dst, int64_t ldd, int rows, int cols, float scale,
                                 int transpose, cudaStream_t s);

@@ -88,14 +88,18 @@ int g_fused_epilogues = 1;  // RoPE / SwiGLU fused into the GEMM and attention e
 // ------------------------------------------------------------------------------------------------
 // LoRA-specific small kernels
 // ------------------------------------------------------------------------------------------------
-// dst[n*r + j] (+)= scale * sum_s part[s*split_stride + (row0+n)*ld + col0 + j]   (fixed order)
-__global__ void lora_gather_kernel(const float* __restrict__ part, int splits, long long split_stride, int ld, int row0,
+// row of output feature n of a target inside its group's weight: plain (row0 + n), or GU-interleaved (wgu: 128 gate rows, then
+// the 128 up rows of the same features, ...; row0 = 0 for gate, 128 for up)
+__host__ __device__ __forceinline__ int target_row(int row0, int n, int gu) { return gu ? row0 + (n >> 7) * 256 + (n & 127) : row0 + n; }
+
+// dst[n*r + j] (+)= scale * sum_s part[s*split_stride + target_row(row0, n, gu)*ld + col0 + j]   (fixed order)
+__global__ void lora_gather_kernel(const float* __restrict__ part, int splits, long long split_stride, int ld, int row0, int gu,
                                    int col0, int rows, int r, float* __restrict__ dst, int accumulate, float scale) {
   const long long total = static_cast<long long>(rows) * r;
   for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < total;
        i += static_cast<long long>(gridDim.x) * blockDim.x) {
     const int n = static_cast<int>(i / r), j = static_cast<int>(i % r);
-    const float* src = part + static_cast<long long>(row0 + n) * ld + col0 + j;
+    const float* src = part + static_cast<long long>(target_row(row0, n, gu)) * ld + col0 + j;
     float s = 0.f;
     for (int k = 0; k < splits; ++k) s += src[k * split_stride];
     s *= scale;
@@ -103,23 +107,47 @@ __global__ void lora_gather_kernel(const float* __restrict__ part, int splits, l
   }
 }
 
+// Adapter groups: the targets that share one input and one frozen weight, so that one LoRA down-projection GEMM serves all
+// of them and their up-projection rides as a K-extension of that weight's GEMM.
+enum { G_ATT = 0, G_GU = 1, G_DN = 2, N_GROUPS = 3 };  // q|k|v -> wqkv (input h1), gate|up -> wgu (h2), down -> wdown (act)
+constexpr int kMaxTargets = 6;                        // q, k, v, gate, up, down (o_proj is not implemented)
+// the linear modules of a decoder layer in HF module order: bit i of dtx_train_cfg.target_mask selects module i
+const char* const kModules[7] = {"q_proj", "k_proj", "v_proj", "o_proj", "gate_proj", "up_proj", "down_proj"};
+constexpr int kModO = 3;
+
 // Per-target geometry of the LoRA adapters inside one layer's block of the flat parameter buffer.
 struct TargetInfo {
-  int row0;        // first row of the target's output features inside wqkv / b_ext
-  int d_out;       // output features (n_heads*128 for q, n_kv_heads*128 for k, v)
-  long long off;   // offset of this target's [A^T (d x r) | B (d_out x r)] inside the layer block
+  int group;       // G_ATT / G_GU / G_DN
+  int gi;          // position inside the group: rank block gi*r of the group's shadows (and input block gi*d_in with dropout)
+  int row0;        // first row of the target's output features inside the group's weight / b_ext (see target_row)
+  int gu;          // rows in the GU-interleaved layout (gate_proj, up_proj)
+  int d_in;        // input features: hidden, or ffn for down_proj
+  int d_out;       // output features (n_heads*128 for q, n_kv_heads*128 for k, v, ffn for gate / up, hidden for down)
+  long long off;   // offset of this target's [A^T (d_in x r) | B (d_out x r)] inside the layer block
 };
 
-// refresh bf16 shadows of all adapters from the fp32 masters.
-//   a_cat[l][(ti*r + j)*KA + a_col0(ti) + c]  = A^T[c*r + j]      (KA = d, a_col0 = 0; with LoRA dropout KA = nt*d, a_col0 = ti*d)
-//   b_ext[l][(row0[ti] + n)*RP + ti*r + j]    = scale * B[n*r + j]
+// bf16 shadows of one group (all layers): a_cat [L][RP][KA], b_ext [L][rows][RP]
+struct GroupInfo {
+  int n = 0;       // enabled targets in the group
+  int ti0 = 0;     // index of its first target among all enabled targets (the dropout mask's target index)
+  int d_in = 0;    // input width of the group
+  int rows = 0;    // output rows of the group's weight (W, 2F, d)
+  int RP = 0;      // n*r rounded up to the 64-wide rank block
+  int KA = 0;      // contraction length of the LoRA down-projection: d_in, or n*d_in with dropout (one dropped copy per target)
+  int split_a = 1, split_b = 1;
+  bf16* a_cat = nullptr;
+  bf16* b_ext = nullptr;
+};
+
+// refresh bf16 shadows of all adapters from the fp32 masters; for target ti of group G:
+//   G.a_cat[l][(gi*r + j)*KA + a_col0 + c]             = A^T[c*r + j]      (a_col0 = 0; with LoRA dropout gi*d_in)
+//   G.b_ext[l][target_row(row0, n, gu)*RP + gi*r + j]  = scale * B[n*r + j]
 struct ShadowArgs {
   const float* params;
-  bf16* a_cat;
-  bf16* b_ext;
-  int L, d, r, RP, nt, KA, W, a_split;
+  int L, r, nt, a_split;
   long long per_layer;
-  TargetInfo tg[3];
+  TargetInfo tg[kMaxTargets];
+  GroupInfo g[N_GROUPS];
   float scale;
 };
 __global__ void lora_shadow_kernel(ShadowArgs a) {
@@ -130,15 +158,18 @@ __global__ void lora_shadow_kernel(ShadowArgs a) {
     long long rem = i - l * a.per_layer;
     int ti = 0;
     while (ti + 1 < a.nt && rem >= a.tg[ti + 1].off) ++ti;
-    rem -= a.tg[ti].off;
+    const TargetInfo& tg = a.tg[ti];
+    const GroupInfo& g = a.g[tg.group];
+    rem -= tg.off;
     const float v = a.params[i];
-    if (rem < static_cast<long long>(a.d) * a.r) {
+    if (rem < static_cast<long long>(tg.d_in) * a.r) {
       const int c = static_cast<int>(rem / a.r), j = static_cast<int>(rem % a.r);
-      a.a_cat[(static_cast<long long>(l) * a.RP + ti * a.r + j) * a.KA + (a.a_split ? ti * a.d : 0) + c] = __float2bfloat16_rn(v);
+      g.a_cat[(static_cast<long long>(l) * g.RP + tg.gi * a.r + j) * g.KA + (a.a_split ? tg.gi * tg.d_in : 0) + c] = __float2bfloat16_rn(v);
     } else {
-      rem -= static_cast<long long>(a.d) * a.r;
+      rem -= static_cast<long long>(tg.d_in) * a.r;
       const int n = static_cast<int>(rem / a.r), j = static_cast<int>(rem % a.r);
-      a.b_ext[(static_cast<long long>(l) * a.W + a.tg[ti].row0 + n) * a.RP + ti * a.r + j] = __float2bfloat16_rn(v * a.scale);
+      g.b_ext[(static_cast<long long>(l) * g.rows + target_row(tg.row0, n, tg.gu)) * g.RP + tg.gi * a.r + j] =
+          __float2bfloat16_rn(v * a.scale);
     }
   }
 }
@@ -146,9 +177,11 @@ __global__ void lora_shadow_kernel(ShadowArgs a) {
 struct Layer {
   // wgu: [2F, d] in the GU-interleaved layout (128 gate rows | 128 up rows per 128 features)
   bf16 *wqkv = nullptr, *wo = nullptr, *wgu = nullptr, *wdown = nullptr, *norm1 = nullptr, *norm2 = nullptr;
-  bf16 *a_cat = nullptr, *b_ext = nullptr;                                               // shadows
-  bf16 *h1 = nullptr, *t = nullptr, *qkv = nullptr, *attn = nullptr, *x_mid = nullptr, *gu = nullptr;  // saved
-  bf16* hd = nullptr;  // LoRA dropout only: [M, nt*d] dropped copies of h1, one per target (peft: one nn.Dropout per module)
+  bf16* a_cat[N_GROUPS] = {nullptr, nullptr, nullptr};  // shadows of the adapter groups (null: group has no target)
+  bf16* b_ext[N_GROUPS] = {nullptr, nullptr, nullptr};
+  bf16* t[N_GROUPS] = {nullptr, nullptr, nullptr};      // saved LoRA down-projections t_g = lora_in * A_cat^T  [M, RP_g]
+  bf16 *h1 = nullptr, *qkv = nullptr, *attn = nullptr, *x_mid = nullptr, *gu = nullptr;  // saved
+  bf16* hd = nullptr;  // LoRA dropout on q/k/v only: [M, n*d] dropped copies of h1, one per target (peft: one nn.Dropout per module)
   float *lse = nullptr, *rstd1 = nullptr, *rstd2 = nullptr;
   // --quantization int4: packed NF4 codes (two per byte) + one fp32 absmax per 64 elements; the bf16 pointers above are then
   // null and the GEMMs read a per-trainer scratch that dequantize() fills right before each launch
@@ -178,7 +211,7 @@ struct dtx_trainer {
   std::vector<void*> allocs;
   size_t bytes_allocated = 0;
 
-  int M = 0, RP = 0, nt = 0;    // M = micro_batch * seq_len: the largest batch this trainer was created for
+  int M = 0, nt = 0;            // M = micro_batch * seq_len: the largest batch this trainer was created for; nt = LoRA targets
   int cur_S = 0, cur_M = 0;     // padded length / token count of the batch being processed (<= seq_len / M)
   int cur_B = 0;                // its rows: micro_batch, or the rows of one length group (SubPlan)
   bool sub_accum = false;       // a later length group of the same micro-batch: gradients and loss add to the earlier groups'
@@ -188,22 +221,22 @@ struct dtx_trainer {
   bool packed = false;          // the batch in d_ids / d_labels is PACKED: sequence b owns rows d_row_start[b] .. d_row_start[b+1])
   bool use_seq_lens = false;    // d_seq_lens holds this batch's true row lengths
   int dq = 0, dkv = 0, W = 0;  // q width (= hidden), k/v width (n_kv_heads*128), packed qkv row width
-  int KA = 0;                  // contraction length of the LoRA down-projection: d, or nt*d with dropout
   bool dropout = false;
-  TargetInfo tg[3];
-  char tg_name[3] = {0, 0, 0};
+  TargetInfo tg[kMaxTargets];   // enabled targets in HF module order
+  int tg_mod[kMaxTargets] = {}; // their HF module index (kModules)
+  GroupInfo grp[N_GROUPS];
   int64_t per_layer = 0, n_train = 0;
   uint64_t fwd_count = 0;      // forward passes so far: seeds the dropout masks
 
   bf16 *embed = nullptr, *lm_head = nullptr, *normf = nullptr;
   std::vector<Layer> layers;
   std::vector<bf16*> xs;  // residual stream, L+1 entries
-  bf16 *a_cat_all = nullptr, *b_ext_all = nullptr;
   float *params = nullptr, *grads = nullptr, *adam_m = nullptr, *adam_v = nullptr;
 
   // transients
   bf16 *h2 = nullptr, *act = nullptr, *dact = nullptr, *dgu = nullptr, *dx_a = nullptr, *dx_b = nullptr, *dh = nullptr,
        *dattn = nullptr, *dqkv = nullptr, *dt = nullptr, *dlogits = nullptr, *glora = nullptr;
+  bf16* hd_mlp = nullptr;  // LoRA dropout on MLP targets: dropped copies of h2 (gate|up) or act (down), rebuilt in the backward pass
   float *logits = nullptr, *rstdf = nullptr, *row_loss = nullptr, *delta = nullptr, *part_b = nullptr, *part_a = nullptr;
   float *d_loss = nullptr, *d_sumsq = nullptr, *d_gnorm = nullptr, *d_scratch = nullptr;
   int32_t *d_ids = nullptr, *d_labels = nullptr, *d_shift = nullptr, *d_nvalid = nullptr, *d_seq_lens = nullptr;
@@ -245,7 +278,6 @@ struct dtx_trainer {
   int64_t base_bytes = 0;
   float2* rope_cs = nullptr;
   float2* rope_cs_t = nullptr;  // the same table transposed to [D/2][S]: coalesced when thread r needs position q0 + r (attention backward epilogues)
-  int split_b = 1, split_a = 1;
 
   // which base tensors have been uploaded: [0] embed, [1] lm_head, [2] final norm, then 9 per layer
   // (q, k, v, o, gate, up, down, norm1, norm2); a step with a hole in this map would train on uninitialised memory
@@ -361,7 +393,7 @@ int pick_split(int m_tiles, int kb_total) {
 int create_buffers(dtx_trainer* t) {
   const dtx_model_cfg& mc = t->mc;
   const dtx_train_cfg& tc = t->tc;
-  const size_t d = mc.hidden, F = mc.ffn, V = mc.vocab, L = mc.n_layers, M = t->M, RP = t->RP, W = t->W, KA = t->KA;
+  const size_t d = mc.hidden, F = mc.ffn, V = mc.vocab, L = mc.n_layers, M = t->M, W = t->W;
   bool ok = true;
   const bool full = t->full;
   if (full) {
@@ -395,10 +427,14 @@ int create_buffers(dtx_trainer* t) {
     t->n_train = static_cast<int64_t>(L * t->layer_used + t->glob_used);
   } else {
     ok = ok && t->alloc(&t->embed, V * d) && t->alloc(&t->lm_head, V * d) && t->alloc(&t->normf, d);
-    ok = ok && t->alloc(&t->a_cat_all, L * RP * KA) && t->alloc(&t->b_ext_all, L * W * RP);
-    if (!ok) return DTX_ERR_CUDA;
-    CKM(cudaMemset(t->a_cat_all, 0, L * RP * KA * sizeof(bf16)));
-    CKM(cudaMemset(t->b_ext_all, 0, L * W * RP * sizeof(bf16)));
+    for (GroupInfo& g : t->grp) {
+      if (!g.n) continue;
+      const size_t na = L * g.RP * g.KA, nb = L * g.rows * g.RP;
+      ok = ok && t->alloc(&g.a_cat, na) && t->alloc(&g.b_ext, nb);
+      if (!ok) return DTX_ERR_CUDA;
+      CKM(cudaMemset(g.a_cat, 0, na * sizeof(bf16)));
+      CKM(cudaMemset(g.b_ext, 0, nb * sizeof(bf16)));
+    }
   }
   t->base_bytes = static_cast<int64_t>((2 * V * d + d) * sizeof(bf16));
   t->loaded.assign(3 + 9 * L, 0);
@@ -414,14 +450,18 @@ int create_buffers(dtx_trainer* t) {
     } else {
       ok = ok && t->alloc(&y.wqkv, W * d) && t->alloc(&y.wo, d * d) && t->alloc(&y.wgu, 2 * F * d) &&
            t->alloc(&y.wdown, d * F) && t->alloc(&y.norm1, d) && t->alloc(&y.norm2, d);
-      y.a_cat = t->a_cat_all + l * RP * KA;
-      y.b_ext = t->b_ext_all + l * W * RP;
-      ok = ok && t->alloc(&y.t, M * RP);
+      for (int gi = 0; gi < N_GROUPS; ++gi) {
+        const GroupInfo& g = t->grp[gi];
+        if (!g.n) continue;
+        y.a_cat[gi] = g.a_cat + l * g.RP * g.KA;
+        y.b_ext[gi] = g.b_ext + l * g.rows * g.RP;
+        ok = ok && t->alloc(&y.t[gi], M * g.RP);
+      }
     }
     t->base_bytes += static_cast<int64_t>((W * d + d * d + 3 * F * d + 2 * d) * sizeof(bf16));
     ok = ok && t->alloc(&y.h1, M * d) && t->alloc(&y.qkv, M * W) &&
          t->alloc(&y.attn, M * d) && t->alloc(&y.x_mid, M * d) && t->alloc(&y.gu, M * 2 * F);
-    if (t->dropout) ok = ok && t->alloc(&y.hd, M * KA);
+    if (t->dropout && t->grp[G_ATT].n) ok = ok && t->alloc(&y.hd, M * t->grp[G_ATT].KA);
     ok = ok && t->alloc(&y.lse, static_cast<size_t>(tc.micro_batch) * mc.n_heads * tc.seq_len) && t->alloc(&y.rstd1, M) &&
          t->alloc(&y.rstd2, M);
   }
@@ -437,16 +477,26 @@ int create_buffers(dtx_trainer* t) {
   }
   ok = ok && t->alloc(&t->h2, M * d) && t->alloc(&t->act, M * F) && t->alloc(&t->dact, M * F) && t->alloc(&t->dgu, M * 2 * F) &&
        t->alloc(&t->dx_a, M * d) && t->alloc(&t->dx_b, M * d) && t->alloc(&t->dh, M * d) && t->alloc(&t->dattn, M * d) &&
-       t->alloc(&t->dqkv, M * W) && (full || t->alloc(&t->dt, M * RP)) && t->alloc(&t->dlogits, M * V) && t->alloc(&t->logits, M * V) &&
+       t->alloc(&t->dqkv, M * W) && t->alloc(&t->dlogits, M * V) && t->alloc(&t->logits, M * V) &&
        t->alloc(&t->rstdf, M) && t->alloc(&t->row_loss, M) &&
        t->alloc(&t->delta, static_cast<size_t>(tc.micro_batch) * mc.n_heads * tc.seq_len);
-  const int kb_tok = (static_cast<int>(M) + 63) / 64;
-  t->split_b = pick_split((static_cast<int>(W) + 127) / 128, kb_tok);
-  t->split_a = pick_split((static_cast<int>(KA) + 127) / 128, kb_tok);
-  if (!full)
-    ok = ok && t->alloc(&t->part_b, static_cast<size_t>(t->split_b) * W * RP) &&
-         t->alloc(&t->part_a, static_cast<size_t>(t->split_a) * KA * RP);
-  if (t->dropout) ok = ok && t->alloc(&t->glora, M * KA);
+  if (!full) {  // per-step LoRA scratch, shared by the groups (the backward pass finishes one group before it starts the next)
+    const int kb_tok = (static_cast<int>(M) + 63) / 64;
+    size_t n_dt = 0, n_pb = 0, n_pa = 0, n_glora = 0, n_hd = 0;
+    for (int gi = 0; gi < N_GROUPS; ++gi) {
+      GroupInfo& g = t->grp[gi];
+      if (!g.n) continue;
+      g.split_b = pick_split((g.rows + 127) / 128, kb_tok);
+      g.split_a = pick_split((g.KA + 127) / 128, kb_tok);
+      n_dt = std::max(n_dt, M * g.RP);
+      n_pb = std::max(n_pb, static_cast<size_t>(g.split_b) * g.rows * g.RP);
+      n_pa = std::max(n_pa, static_cast<size_t>(g.split_a) * g.KA * g.RP);
+      n_glora = std::max(n_glora, M * g.KA);
+      if (gi != G_ATT) n_hd = std::max(n_hd, M * g.KA);
+    }
+    ok = ok && t->alloc(&t->dt, n_dt) && t->alloc(&t->part_b, n_pb) && t->alloc(&t->part_a, n_pa);
+    if (t->dropout) ok = ok && t->alloc(&t->glora, n_glora) && (n_hd == 0 || t->alloc(&t->hd_mlp, n_hd));
+  }
   ok = ok && t->alloc(&t->d_loss, 4) && t->alloc(&t->d_sumsq, 4) && t->alloc(&t->d_gnorm, 4) && t->alloc(&t->d_scratch, 1024);
   ok = ok && t->alloc(&t->d_ids, M) && t->alloc(&t->d_labels, M) && t->alloc(&t->d_shift, M) && t->alloc(&t->d_nvalid, 4);
   ok = ok && t->alloc(&t->d_row_map, M) && t->alloc(&t->d_valid_idx, M);
@@ -481,18 +531,13 @@ int create_buffers(dtx_trainer* t) {
 int refresh_shadows(dtx_trainer* t) {
   ShadowArgs a;
   a.params = t->params;
-  a.a_cat = t->a_cat_all;
-  a.b_ext = t->b_ext_all;
   a.L = t->mc.n_layers;
-  a.d = t->mc.hidden;
   a.r = t->tc.lora_r;
-  a.RP = t->RP;
   a.nt = t->nt;
-  a.KA = t->KA;
-  a.W = t->W;
   a.a_split = t->dropout ? 1 : 0;
   a.per_layer = t->per_layer;
-  for (int i = 0; i < 3; ++i) a.tg[i] = t->tg[i];
+  for (int i = 0; i < kMaxTargets; ++i) a.tg[i] = t->tg[i];
+  for (int i = 0; i < N_GROUPS; ++i) a.g[i] = t->grp[i];
   a.scale = t->tc.lora_alpha / static_cast<float>(t->tc.lora_r);
   long long total = t->n_train;
   int grid = static_cast<int>((total + 255) / 256);
@@ -602,21 +647,45 @@ int reduce_scatter_block(dtx_trainer* t, bf16* block, int64_t elems, int ev_idx)
 int fwd_bwd(dtx_trainer* t, bool backward) {
   const dtx_model_cfg& mc = t->mc;
   const dtx_train_cfg& tc = t->tc;
-  const int d = mc.hidden, F = mc.ffn, V = mc.vocab, L = mc.n_layers, M = t->cur_M, RP = t->RP, H = mc.n_heads, D = mc.head_dim;
+  const int d = mc.hidden, F = mc.ffn, V = mc.vocab, L = mc.n_layers, M = t->cur_M, H = mc.n_heads, D = mc.head_dim;
   const int Hkv = mc.n_kv_heads, W = t->W;
   const int B = t->cur_B, S = t->cur_S;
   const int32_t* seq_lens = t->use_seq_lens ? t->d_seq_lens : nullptr;
   const int kb_tok = (M + 63) / 64;
-  const int split_b = std::min(t->split_b, pick_split((W + 127) / 128, kb_tok));
-  const int split_a = std::min(t->split_a, pick_split((t->KA + 127) / 128, kb_tok));
   cudaStream_t s = t->stream;
   const float att_scale = 1.0f / sqrtf(static_cast<float>(D));
   const bool fused = g_fused_epilogues && M > 128 && ((t->dq + t->dkv) % 256 == 0) && (W % 256 == 0);  // whole 256-column tiles
   const bool lora = !t->full;    // full-parameter SFT: no adapters, every weight gets a gradient
+  const GroupInfo &ga = t->grp[G_ATT], &gg = t->grp[G_GU], &gd = t->grp[G_DN];
+  const bool lora_att = lora && ga.n > 0, lora_gu = lora && gg.n > 0, lora_dn = lora && gd.n > 0;
   bool in_backward = false;      // which half of the step asks for a base weight (prefetch order of the NF4 expansion)
-  const bool drop = lora && t->dropout;  // adapters laid out for per-target dropped inputs (KA = nt*d)
+  const bool drop = lora && t->dropout;  // adapters laid out for per-target dropped inputs (KA = n*d_in)
   const float p_drop = backward ? tc.lora_dropout : 0.f;  // eval (model.eval()) runs the same path with p = 0
   t->fwd_count += 1;
+  // dropout key of group g in layer l: the mask of a target is indexed by its position among ALL enabled targets, and the
+  // kernels add (position inside the group) * G to the key - so the group's offset goes into the key
+  auto group_key = [&](int l, const GroupInfo& g) { return dropout_key(t, l) + static_cast<uint64_t>(g.ti0) * 0x9E3779B97F4A7C15ull; };
+  // t_g = lora_in * A_cat^T  [M, RP]: the LoRA down-projection of every target of a group in one GEMM
+  auto lora_down = [&](const GroupInfo& G, const bf16* in, const bf16* a_cat, bf16* out) {
+    GemmArgs g;
+    g.A = in; g.lda = G.KA; g.B = a_cat; g.ldb = G.KA; g.C = out; g.ldc = G.RP;
+    g.M = M; g.N = G.RP; g.K = G.KA; g.epilogue = EPI_BF16; g.block_n = 64;
+    return gemm_bf16(g, s);
+  };
+  // dt = dY * B_ext  [M, RP]  (dY: gradient of the group's output, [M, rows])
+  auto lora_dt = [&](const GroupInfo& G, const bf16* dY, const bf16* b_ext) {
+    GemmArgs g;
+    g.A = dY; g.lda = G.rows; g.B = b_ext; g.ldb = G.RP; g.b_mn_major = 1; g.C = t->dt; g.ldc = G.RP;
+    g.M = M; g.N = G.RP; g.K = G.rows; g.epilogue = EPI_BF16; g.block_n = 64;
+    return gemm_bf16(g, s);
+  };
+  // glora = dt * A_cat  [M, KA]: the LoRA branch's input gradient before the dropout masks (one block per target)
+  auto lora_dx = [&](const GroupInfo& G, const bf16* a_cat) {
+    GemmArgs g;
+    g.A = t->dt; g.lda = G.RP; g.B = a_cat; g.ldb = G.KA; g.b_mn_major = 1; g.C = t->glora; g.ldc = G.KA;
+    g.M = M; g.N = G.KA; g.K = G.RP; g.epilogue = EPI_BF16;
+    return gemm_bf16(g, s);
+  };
 
   wait_weights(t, L);  // globals (embedding, lm_head, final norm)
   CK(embedding_fwd(t->d_ids, t->embed, t->xs[0], M, d, V, s), 1);
@@ -625,21 +694,16 @@ int fwd_bwd(dtx_trainer* t, bool backward) {
     wait_weights(t, l);
     CK(rmsnorm_fwd(t->xs[l], y.norm1, y.h1, y.rstd1, M, d, mc.rms_eps, s), 1);
     const bf16* lora_in = y.h1;
-    if (drop) {  // peft: lora_A(lora_dropout(x)) with one nn.Dropout per wrapped module -> one dropped copy per target
-      CK(lora_dropout_fwd(y.h1, y.hd, M, d, t->nt, p_drop, dropout_key(t, l), s), 1);
+    if (drop && lora_att) {  // peft: lora_A(lora_dropout(x)) with one nn.Dropout per wrapped module -> one dropped copy per target
+      CK(lora_dropout_fwd(y.h1, y.hd, M, d, ga.n, p_drop, dropout_key(t, l), s), 1);
       lora_in = y.hd;
     }
-    if (lora) {  // LoRA down-projection of all targets at once: t = lora_in * A_cat^T   [M, RP]
-      GemmArgs g;
-      g.A = lora_in; g.lda = t->KA; g.B = y.a_cat; g.ldb = t->KA; g.C = y.t; g.ldc = RP;
-      g.M = M; g.N = RP; g.K = t->KA; g.epilogue = EPI_BF16; g.block_n = 64;
-      CK(gemm_bf16(g, s), 1);
-    }
+    if (lora_att) CK(lora_down(ga, lora_in, y.a_cat[G_ATT], y.t[G_ATT]), 1);  // t = lora_in * A_cat^T   [M, RP]
     {  // qkv = h1 * Wqkv^T + t * B_ext^T : base projection and LoRA up-projection in one TMEM accumulator
       BASEW(W_QKV, wqkv);
       GemmArgs g;
       g.A = y.h1; g.lda = d; g.B = wqkv; g.ldb = d;
-      if (lora) { g.A2 = y.t; g.lda2 = RP; g.B2 = y.b_ext; g.ldb2 = RP; g.K2 = RP; }
+      if (lora_att) { g.A2 = y.t[G_ATT]; g.lda2 = ga.RP; g.B2 = y.b_ext[G_ATT]; g.ldb2 = ga.RP; g.K2 = ga.RP; }
       g.C = y.qkv; g.ldc = W; g.M = M; g.N = W; g.K = d; g.epilogue = EPI_BF16;
       if (fused) {  // rotary embedding of q and k applied to the fp32 accumulator in the epilogue
         g.epilogue = EPI_ROPE; g.rope_cs = t->rope_cs; g.rope_S = S; g.rope_cols = t->dq + t->dkv;
@@ -664,10 +728,19 @@ int fwd_bwd(dtx_trainer* t, bool backward) {
       CK(gemm_bf16(g, s), 1);
     }
     CK(rmsnorm_fwd(y.x_mid, y.norm2, t->h2, y.rstd2, M, d, mc.rms_eps, s), 1);
-    {  // [gate | up] = h2 * Wgu^T
+    if (lora_gu) {  // t_gu = h2 * A_gu^T  (h2 and its dropped copies are per-step scratch: the backward pass rebuilds them)
+      const bf16* in = t->h2;
+      if (drop) {
+        CK(lora_dropout_fwd(t->h2, t->hd_mlp, M, d, gg.n, p_drop, group_key(l, gg), s), 1);
+        in = t->hd_mlp;
+      }
+      CK(lora_down(gg, in, y.a_cat[G_GU], y.t[G_GU]), 1);
+    }
+    {  // [gate | up] = h2 * Wgu^T + t_gu * B_gu^T  (B_gu rows GU-interleaved like Wgu: gate and up of a feature share a tile)
       BASEW(W_GU, wgu);
       GemmArgs g;
       g.A = t->h2; g.lda = d; g.B = wgu; g.ldb = d; g.C = y.gu; g.ldc = 2 * F;
+      if (lora_gu) { g.A2 = y.t[G_GU]; g.lda2 = gg.RP; g.B2 = y.b_ext[G_GU]; g.ldb2 = gg.RP; g.K2 = gg.RP; }
       g.M = M; g.N = 2 * F; g.K = d; g.epilogue = EPI_BF16;
       if (fused) {  // silu(gate) * up computed from the accumulator tile ([gate 128 | up 128] interleaved layout)
         g.epilogue = EPI_SWIGLU_FWD; g.aux = t->act; g.ld_aux = F;
@@ -675,10 +748,19 @@ int fwd_bwd(dtx_trainer* t, bool backward) {
       CK(gemm_bf16(g, s), 1);
     }
     if (!fused) CK(swiglu_fwd(y.gu, t->act, M, F, 1, s), 1);
-    {  // x_next = x_mid + act * Wdown^T
+    if (lora_dn) {  // t_dn = act * A_dn^T  (K = F)
+      const bf16* in = t->act;
+      if (drop) {
+        CK(lora_dropout_fwd(t->act, t->hd_mlp, M, F, 1, p_drop, group_key(l, gd), s), 1);
+        in = t->hd_mlp;
+      }
+      CK(lora_down(gd, in, y.a_cat[G_DN], y.t[G_DN]), 1);
+    }
+    {  // x_next = x_mid + act * Wdown^T + t_dn * B_dn^T
       BASEW(W_DOWN, wdown);
       GemmArgs g;
       g.A = t->act; g.lda = F; g.B = wdown; g.ldb = F; g.C = t->xs[l + 1]; g.ldc = d; g.R = y.x_mid; g.ldr = d;
+      if (lora_dn) { g.A2 = y.t[G_DN]; g.lda2 = gd.RP; g.B2 = y.b_ext[G_DN]; g.ldb2 = gd.RP; g.K2 = gd.RP; }
       g.M = M; g.N = d; g.K = F; g.epilogue = EPI_BF16_ADD;
       CK(gemm_bf16(g, s), 1);
     }
@@ -718,6 +800,41 @@ int fwd_bwd(dtx_trainer* t, bool backward) {
     g.epilogue = accumulate ? EPI_BF16_ADD : EPI_BF16; g.R = accumulate ? dW : nullptr; g.ldr = n_in;
     return gemm_bf16(g, s);
   };
+  // adapter gradients of group gi in layer l: grad of B_ext (all rows) dY^T * t_g [rows, RP] and grad of A_cat^T lora_in^T * dt
+  // [KA, RP], both split over tokens, then gathered per target into the flat gradient.  dA^T = lora_in^T (dy * sB) (the scale
+  // rides in B_ext); dB = s * dy^T t (t is unscaled, so the scale is applied by the gather).
+  auto lora_wgrad = [&](int l, int gi, const bf16* dY, const bf16* lora_in) -> int {
+    const GroupInfo& G = t->grp[gi];
+    const int split_b = std::min(G.split_b, pick_split((G.rows + 127) / 128, kb_tok));
+    const int split_a = std::min(G.split_a, pick_split((G.KA + 127) / 128, kb_tok));
+    {
+      GemmArgs g;
+      g.A = dY; g.lda = G.rows; g.a_mn_major = 1; g.B = t->layers[l].t[gi]; g.ldb = G.RP; g.b_mn_major = 1;
+      g.C = t->part_b; g.ldc = G.RP; g.M = G.rows; g.N = G.RP; g.K = M; g.epilogue = EPI_F32; g.split_k = split_b;
+      g.block_n = 64;
+      CK(gemm_bf16(g, s), 1);
+    }
+    {
+      GemmArgs g;
+      g.A = lora_in; g.lda = G.KA; g.a_mn_major = 1; g.B = t->dt; g.ldb = G.RP; g.b_mn_major = 1;
+      g.C = t->part_a; g.ldc = G.RP; g.M = G.KA; g.N = G.RP; g.K = M; g.epilogue = EPI_F32; g.split_k = split_a;
+      g.block_n = 64;
+      CK(gemm_bf16(g, s), 1);
+    }
+    const int r = tc.lora_r;
+    for (int ti = G.ti0; ti < G.ti0 + G.n; ++ti) {  // the targets of a group are consecutive in HF module order
+      const TargetInfo& tg = t->tg[ti];
+      float* gl = t->grads + static_cast<int64_t>(l) * t->per_layer + tg.off;
+      lora_gather_kernel<<<(tg.d_in * r + 255) / 256, 256, 0, s>>>(t->part_a, split_a, static_cast<long long>(G.KA) * G.RP, G.RP,
+                                                                 drop ? tg.gi * tg.d_in : 0, 0, tg.gi * r, tg.d_in, r, gl, accumulate, 1.0f);
+      lora_gather_kernel<<<(tg.d_out * r + 255) / 256, 256, 0, s>>>(t->part_b, split_b, static_cast<long long>(G.rows) * G.RP, G.RP,
+                                                                  tg.row0, tg.gu, tg.gi * r, tg.d_out, r,
+                                                                  gl + static_cast<int64_t>(tg.d_in) * r, accumulate,
+                                                                  tc.lora_alpha / static_cast<float>(r));
+      CK(cudaGetLastError(), 2);
+    }
+    return DTX_OK;
+  };
   bf16* gglob = t->full ? t->g_flat + static_cast<int64_t>(L) * t->layer_elems : nullptr;
   if (t->full) {  // lm_head weight gradient (h2 still holds the final-norm output) and the final norm's weight gradient
     CK(dw_gemm(t->dlogits, V, t->h2, d, gglob + t->goff_lm), 1);
@@ -739,28 +856,63 @@ int fwd_bwd(dtx_trainer* t, bool backward) {
       CK(swiglu_fwd(y.gu, t->act, M, F, 1, s), 1);
       CK(dw_gemm(cur, d, t->act, F, gl_w + t->off_wdown), 1);
     }
-    {  // dact = dx * Wdown ; fused: d[gate|up] straight from the accumulator, dact never touches HBM
+    if (lora_dn) CK(lora_dt(gd, cur, y.b_ext[G_DN]), 1);  // dt_dn = dx * B_dn  [M, RP_dn]
+    // with dropout the LoRA branch's input gradient is masked: it cannot ride in the dact GEMM's accumulator
+    const bool dn_dropped = lora_dn && drop;
+    {  // dact = dx * Wdown (+ dt_dn * A_dn) ; fused: d[gate|up] straight from the accumulator, dact never touches HBM
       BASEW(W_DOWN, wdown);
       GemmArgs g;
       g.A = cur; g.lda = d; g.B = wdown; g.ldb = F; g.b_mn_major = 1; g.C = t->dact; g.ldc = F;
+      if (lora_dn && !drop) { g.A2 = t->dt; g.lda2 = gd.RP; g.B2 = y.a_cat[G_DN]; g.ldb2 = gd.KA; g.K2 = gd.RP; }
       g.M = M; g.N = F; g.K = d; g.epilogue = EPI_BF16;
-      if (fused) {
+      if (fused && !dn_dropped) {
         g.epilogue = EPI_SWIGLU_BWD; g.C = t->dgu; g.ldc = 2 * F; g.aux = y.gu; g.ld_aux = 2 * F;
       }
       CK(gemm_bf16(g, s), 1);
     }
-    if (!fused) CK(swiglu_bwd(t->dact, y.gu, t->dgu, M, F, 1, s), 1);
-    {  // dh2 = [dgate | dup] * [Wg ; Wu]
+    if (dn_dropped) {  // d(act) = dact + mask o (dt_dn * A_dn) / (1 - p) and the SwiGLU backward in one pass
+      CK(lora_dx(gd, y.a_cat[G_DN]), 1);
+      CK(swiglu_bwd_lora_dropout(t->dact, t->glora, y.gu, t->dgu, M, F, 1, p_drop, group_key(l, gd), s), 1);
+    } else if (!fused) {
+      CK(swiglu_bwd(t->dact, y.gu, t->dgu, M, F, 1, s), 1);
+    }
+    if (lora_dn) {  // dB_dn = dx^T t_dn, dA_dn = act^T dt_dn: act = silu(gate) * up recomputed from the saved gate|up
+      CK(swiglu_fwd(y.gu, t->act, M, F, 1, s), 1);
+      const bf16* in = t->act;
+      if (drop) {
+        CK(lora_dropout_fwd(t->act, t->hd_mlp, M, F, 1, p_drop, group_key(l, gd), s), 1);
+        in = t->hd_mlp;
+      }
+      int rc = lora_wgrad(l, G_DN, cur, in);
+      if (rc) return rc;
+    }
+    if (lora_gu) CK(lora_dt(gg, t->dgu, y.b_ext[G_GU]), 1);  // dt_gu = d[gate|up] * B_gu  [M, RP_gu]
+    {  // dh2 = [dgate | dup] * [Wg ; Wu] (+ dt_gu * A_gu)
       BASEW(W_GU, wgu);
       GemmArgs g;
       g.A = t->dgu; g.lda = 2 * F; g.B = wgu; g.ldb = d; g.b_mn_major = 1; g.C = t->dh; g.ldc = d;
+      if (lora_gu && !drop) { g.A2 = t->dt; g.lda2 = gg.RP; g.B2 = y.a_cat[G_GU]; g.ldb2 = gg.KA; g.K2 = gg.RP; }
       g.M = M; g.N = d; g.K = 2 * F; g.epilogue = EPI_BF16;
       CK(gemm_bf16(g, s), 1);
     }
-    if (t->full) {  // dWgu = d[gate|up]^T * h2 (h2 = norm2(x_mid) recomputed) and the norm's own weight gradient
+    if (lora_gu && drop) {  // dh2 += sum_t mask_t o (dt_t * A_t) / (1 - p)
+      CK(lora_dx(gg, y.a_cat[G_GU]), 1);
+      CK(lora_dropout_bwd_add(t->dh, t->glora, M, d, gg.n, p_drop, group_key(l, gg), s), 1);
+    }
+    if (t->full || lora_gu)  // h2 = norm2(x_mid) recomputed: dWgu / dA_gu contract it over the tokens
       CK(rmsnorm_fwd(y.x_mid, y.norm2, t->h2, nullptr, M, d, mc.rms_eps, s), 1);
+    if (t->full) {  // dWgu = d[gate|up]^T * h2 and the norm's own weight gradient
       CK(dw_gemm(t->dgu, 2 * F, t->h2, d, gl_w + t->off_wgu), 1);
       CK(rmsnorm_dw(t->dh, y.x_mid, y.rstd2, M, d, t->ndw_scratch, gl_w + t->off_n2, accumulate, s), 2);
+    }
+    if (lora_gu) {  // dB_gu = d[gate|up]^T t_gu (rows gathered out of the interleaved layout), dA_gu = h2^T dt_gu
+      const bf16* in = t->h2;
+      if (drop) {
+        CK(lora_dropout_fwd(t->h2, t->hd_mlp, M, d, gg.n, p_drop, group_key(l, gg), s), 1);
+        in = t->hd_mlp;
+      }
+      int rc = lora_wgrad(l, G_GU, t->dgu, in);
+      if (rc) return rc;
     }
     CK(rmsnorm_bwd(t->dh, y.x_mid, y.norm2, y.rstd2, cur, other, M, d, s), 1);  // other = d x_mid
     {  // dattn = dx_mid * Wo
@@ -785,12 +937,7 @@ int fwd_bwd(dtx_trainer* t, bool backward) {
       CK(attn_bwd(a, s), attn_bwd_launches());
       if (!rope_in_attn) CK(rope_qk_inplace_table(t->dqkv, t->rope_cs, B, S, H + Hkv, W, D, 1, s), 1);
     }
-    if (lora) {  // dt = dqkv * B_ext   [M, RP]
-      GemmArgs g;
-      g.A = t->dqkv; g.lda = W; g.B = y.b_ext; g.ldb = RP; g.b_mn_major = 1; g.C = t->dt; g.ldc = RP;
-      g.M = M; g.N = RP; g.K = W; g.epilogue = EPI_BF16; g.block_n = 64;
-      CK(gemm_bf16(g, s), 1);
-    }
+    if (lora_att) CK(lora_dt(ga, t->dqkv, y.b_ext[G_ATT]), 1);  // dt = dqkv * B_ext   [M, RP]
     if (t->full) CK(dw_gemm(t->dqkv, W, y.h1, d, gl_w), 1);  // dWqkv = dqkv^T * h1 (dqkv already carries the inverse rotary)
     // LoRA: layer 0's input gradient has no consumer (the embedding is frozen, SURVEY §8a): its dh1 GEMM, the dropout-branch
     // gradient and the norm-1 backward are skipped.  Full-parameter SFT trains the embedding and needs them.
@@ -799,45 +946,18 @@ int fwd_bwd(dtx_trainer* t, bool backward) {
       BASEW(W_QKV, wqkv);
       GemmArgs g;
       g.A = t->dqkv; g.lda = W; g.B = wqkv; g.ldb = d; g.b_mn_major = 1;
-      if (lora && !drop) { g.A2 = t->dt; g.lda2 = RP; g.B2 = y.a_cat; g.ldb2 = t->KA; g.K2 = RP; }
+      if (lora_att && !drop) { g.A2 = t->dt; g.lda2 = ga.RP; g.B2 = y.a_cat[G_ATT]; g.ldb2 = ga.KA; g.K2 = ga.RP; }
       g.C = t->dh; g.ldc = d; g.M = M; g.N = d; g.K = W; g.epilogue = EPI_BF16;
       CK(gemm_bf16(g, s), 1);
     }
-    if (drop && need_dx) {  // dh1 += sum_t mask_t o (dt_t * A_t) / (1 - p): the masks are regenerated from the counter-based RNG
-      GemmArgs g;
-      g.A = t->dt; g.lda = RP; g.B = y.a_cat; g.ldb = t->KA; g.b_mn_major = 1; g.C = t->glora; g.ldc = t->KA;
-      g.M = M; g.N = t->KA; g.K = RP; g.epilogue = EPI_BF16;
-      CK(gemm_bf16(g, s), 1);
-      CK(lora_dropout_bwd_add(t->dh, t->glora, M, d, t->nt, p_drop, dropout_key(t, l), s), 1);
+    if (lora_att && drop && need_dx) {  // dh1 += sum_t mask_t o (dt_t * A_t) / (1 - p): the masks are regenerated from the counter-based RNG
+      CK(lora_dx(ga, y.a_cat[G_ATT]), 1);
+      CK(lora_dropout_bwd_add(t->dh, t->glora, M, d, ga.n, p_drop, dropout_key(t, l), s), 1);
     }
-    if (lora) {
-    {  // grad of B_ext (all rows): dqkv^T * t   [W, RP], split over tokens
-      GemmArgs g;
-      g.A = t->dqkv; g.lda = W; g.a_mn_major = 1; g.B = y.t; g.ldb = RP; g.b_mn_major = 1;
-      g.C = t->part_b; g.ldc = RP; g.M = W; g.N = RP; g.K = M; g.epilogue = EPI_F32; g.split_k = split_b;
-      g.block_n = 64;
-      CK(gemm_bf16(g, s), 1);
+    if (lora_att) {
+      int rc = lora_wgrad(l, G_ATT, t->dqkv, drop ? y.hd : y.h1);
+      if (rc) return rc;
     }
-    {  // grad of A_cat^T: lora_in^T * dt   [KA, RP]
-      GemmArgs g;
-      g.A = drop ? y.hd : y.h1; g.lda = t->KA; g.a_mn_major = 1; g.B = t->dt; g.ldb = RP; g.b_mn_major = 1;
-      g.C = t->part_a; g.ldc = RP; g.M = t->KA; g.N = RP; g.K = M; g.epilogue = EPI_F32; g.split_k = split_a;
-      g.block_n = 64;
-      CK(gemm_bf16(g, s), 1);
-    }
-    const int r = tc.lora_r;
-    for (int ti = 0; ti < t->nt; ++ti) {
-      float* gl = t->grads + static_cast<int64_t>(l) * t->per_layer + t->tg[ti].off;
-      const int d_out = t->tg[ti].d_out;
-      // dA^T = lora_in^T (dy * sB)  (the scale rides in B_ext);  dB = s * dy^T t  (t is unscaled, so the scale is applied here)
-      lora_gather_kernel<<<(d * r + 255) / 256, 256, 0, s>>>(t->part_a, split_a, static_cast<long long>(t->KA) * RP, RP,
-                                                            drop ? ti * d : 0, ti * r, d, r, gl, accumulate, 1.0f);
-      lora_gather_kernel<<<(d_out * r + 255) / 256, 256, 0, s>>>(t->part_b, split_b, static_cast<long long>(W) * RP, RP,
-                                                                t->tg[ti].row0, ti * r, d_out, r, gl + static_cast<int64_t>(d) * r,
-                                                                accumulate, tc.lora_alpha / static_cast<float>(r));
-      CK(cudaGetLastError(), 2);
-    }
-    }  // lora
     if (t->full) CK(rmsnorm_dw(t->dh, t->xs[l], y.rstd1, M, d, t->ndw_scratch, gl_w + t->off_n1, accumulate, s), 2);
     if (need_dx) CK(rmsnorm_bwd(t->dh, t->xs[l], y.norm1, y.rstd1, other, cur, M, d, s), 1);  // cur = d x_in
     if (t->full && t->rs_now && t->world > 1) {  // this layer's gradients are final: reduce-scatter them while the backward pass goes on
@@ -1199,9 +1319,16 @@ void to_f32_host(const void* src, int dtype, size_t n, std::vector<float>& out) 
   }
 }
 
-int target_index(const dtx_trainer* t, char which) {  // 'q','k','v' -> index among enabled targets or -1
-  for (int i = 0; i < t->nt; ++i)
-    if (t->tg_name[i] == which) return i;
+// index among the enabled targets of the LoRA module named in `rest` ("self_attn.q_proj.lora_A.weight", "mlp.down_proj...."),
+// or -1 when it names no enabled target
+int target_index(const dtx_trainer* t, const char* rest) {
+  int mod = -1;
+  for (int m = 0; m < 7 && mod < 0; ++m) {
+    const char* p = strstr(rest, kModules[m]);
+    if (p && (p == rest || p[-1] == '.')) mod = m;  // a whole path component, not the tail of another name
+  }
+  for (int i = 0; i < t->nt && mod >= 0; ++i)
+    if (t->tg_mod[i] == mod) return i;
   return -1;
 }
 
@@ -1264,8 +1391,12 @@ int32_t dtx_trainer_create(const dtx_model_cfg* mc, const dtx_train_cfg* tc, int
   if (tc->seq_len > mc->max_seq) return bad("seq_len exceeds max_seq");
   if (!tc->full_finetune && (tc->lora_r <= 0 || tc->lora_r % 8)) return bad("lora_r must be a positive multiple of 8");
   if (tc->lora_dropout < 0.0f || tc->lora_dropout >= 1.0f) return bad("lora_dropout must be in [0, 1)");
-  if (!tc->full_finetune && ((tc->target_mask & ~(DTX_TARGET_Q | DTX_TARGET_K | DTX_TARGET_V)) || tc->target_mask == 0))
-    { g_error = "lora_target must be a non-empty subset of q_proj,k_proj,v_proj"; return DTX_ERR_UNSUPPORTED; }
+  const uint32_t implemented = DTX_TARGET_Q | DTX_TARGET_K | DTX_TARGET_V | DTX_TARGET_GATE | DTX_TARGET_UP | DTX_TARGET_DOWN;
+  if (!tc->full_finetune && ((tc->target_mask & ~implemented) || tc->target_mask == 0)) {
+    g_error = "lora_target must be a non-empty subset of q_proj,k_proj,v_proj,gate_proj,up_proj,down_proj "
+              "(o_proj is the one linear module whose adapter is not implemented)";
+    return DTX_ERR_UNSUPPORTED;
+  }
   if (world < 1 || rank < 0 || rank >= world) return bad("bad rank/world");
   if (world > 1 && !nccl_unique_id) return bad("world > 1 needs an NCCL unique id");
 
@@ -1296,22 +1427,37 @@ int32_t dtx_trainer_create(const dtx_model_cfg* mc, const dtx_train_cfg* tc, int
   t->nt = 0;
   t->per_layer = 0;
   if (!t->full) {
-    const unsigned bits[3] = {DTX_TARGET_Q, DTX_TARGET_K, DTX_TARGET_V};
-    const char names[3] = {'q', 'k', 'v'};
-    const int row0[3] = {0, t->dq, t->dq + t->dkv};
-    const int dout[3] = {t->dq, t->dkv, t->dkv};
-    for (int i = 0; i < 3; ++i)
-      if (tc->target_mask & bits[i]) {
-        t->tg[t->nt].row0 = row0[i];
-        t->tg[t->nt].d_out = dout[i];
-        t->tg[t->nt].off = t->per_layer;
-        t->tg_name[t->nt] = names[i];
-        t->per_layer += static_cast<int64_t>(mc->hidden + dout[i]) * tc->lora_r;
-        ++t->nt;
-      }
+    // per-layer block of the flat parameter buffer: [A^T | B] of every enabled target in HF module order
+    const int d = mc->hidden, F = mc->ffn;
+    struct Mod { int group, row0, gu, d_in, d_out; };
+    const Mod mods[7] = {{G_ATT, 0, 0, d, t->dq},     {G_ATT, t->dq, 0, d, t->dkv}, {G_ATT, t->dq + t->dkv, 0, d, t->dkv},
+                         {-1, 0, 0, 0, 0},             {G_GU, 0, 1, d, F},            {G_GU, 128, 1, d, F},
+                         {G_DN, 0, 0, F, d}};
+    const int rows[N_GROUPS] = {t->W, 2 * F, d};
+    for (int m = 0; m < 7; ++m) {
+      if (m == kModO || !(tc->target_mask & (1u << m))) continue;
+      GroupInfo& g = t->grp[mods[m].group];
+      if (g.n == 0) g.ti0 = t->nt;
+      TargetInfo& tg = t->tg[t->nt];
+      tg.group = mods[m].group;
+      tg.gi = g.n++;
+      tg.row0 = mods[m].row0;
+      tg.gu = mods[m].gu;
+      tg.d_in = mods[m].d_in;
+      tg.d_out = mods[m].d_out;
+      tg.off = t->per_layer;
+      t->tg_mod[t->nt] = m;
+      t->per_layer += static_cast<int64_t>(tg.d_in + tg.d_out) * tc->lora_r;
+      ++t->nt;
+    }
+    for (int gi = 0; gi < N_GROUPS; ++gi) {
+      GroupInfo& g = t->grp[gi];
+      g.d_in = gi == G_DN ? F : d;
+      g.rows = rows[gi];
+      g.RP = ((g.n * tc->lora_r + 63) / 64) * 64;
+      g.KA = t->dropout ? g.n * g.d_in : g.d_in;
+    }
   }
-  t->RP = ((t->nt * tc->lora_r + 63) / 64) * 64;
-  t->KA = t->dropout ? t->nt * mc->hidden : mc->hidden;
   t->n_train = static_cast<int64_t>(mc->n_layers) * t->per_layer;
   t->cur_S = tc->seq_len;
   t->cur_M = t->M;
@@ -1430,26 +1576,22 @@ int32_t dtx_load_tensor(dtx_trainer* t, const char* name, const void* host, int3
   uint8_t* lmap = t->loaded.data() + 3 + 9 * static_cast<size_t>(layer);
   const bool is_lora_a = strstr(rest, "lora_A") != nullptr, is_lora_b = strstr(rest, "lora_B") != nullptr;
   if (is_lora_a || is_lora_b) {
-    char which = 0;
-    if (strstr(rest, "q_proj")) which = 'q';
-    else if (strstr(rest, "k_proj")) which = 'k';
-    else if (strstr(rest, "v_proj")) which = 'v';
-    const int ti = which ? target_index(t, which) : -1;
+    const int ti = target_index(t, rest);
     if (ti < 0) return t->fail(DTX_ERR_INVALID, "%s: module is not a LoRA target", name);
     float* base = t->params + static_cast<int64_t>(layer) * t->per_layer + t->tg[ti].off;
-    const int64_t d_out = t->tg[ti].d_out;
+    const int64_t d_in = t->tg[ti].d_in, d_out = t->tg[ti].d_out;
     std::vector<float> f;
-    if (is_lora_a) {  // [r, d] -> stored transposed [d, r]
-      if (!expect(r, d)) return t->fail(DTX_ERR_INVALID, "%s: expected [%lld,%lld]", name, (long long)r, (long long)d);
-      to_f32_host(host, dtype, r * d, f);
-      std::vector<float> tr(d * r);
+    if (is_lora_a) {  // [r, d_in] -> stored transposed [d_in, r]
+      if (!expect(r, d_in)) return t->fail(DTX_ERR_INVALID, "%s: expected [%lld,%lld]", name, (long long)r, (long long)d_in);
+      to_f32_host(host, dtype, r * d_in, f);
+      std::vector<float> tr(d_in * r);
       for (int64_t j = 0; j < r; ++j)
-        for (int64_t c = 0; c < d; ++c) tr[c * r + j] = f[j * d + c];
+        for (int64_t c = 0; c < d_in; ++c) tr[c * r + j] = f[j * d_in + c];
       CKM(upload_sync(base, tr.data(), tr.size() * 4, t->stream));
     } else {
       if (!expect(d_out, r)) return t->fail(DTX_ERR_INVALID, "%s: expected [%lld,%lld]", name, (long long)d_out, (long long)r);
       to_f32_host(host, dtype, d_out * r, f);
-      CKM(upload_sync(base + d * r, f.data(), f.size() * 4, t->stream));
+      CKM(upload_sync(base + d_in * r, f.data(), f.size() * 4, t->stream));
     }
     t->have_lora = true;
     int rc = refresh_shadows(t);
@@ -1570,10 +1712,9 @@ int32_t dtx_init_lora(dtx_trainer* t, uint64_t seed) {
   if (!t) return DTX_ERR_INVALID;
   if (t->full) return t->fail(DTX_ERR_STATE, "init_lora: this trainer was created for full-parameter SFT (no adapters)");
   cudaSetDevice(t->device);
-  const int64_t d = t->mc.hidden, r = t->tc.lora_r;
+  const int64_t r = t->tc.lora_r;
   std::vector<float> host(t->n_train, 0.f);
   // peft 0.5.0 LoraLayer.reset_lora_parameters: kaiming_uniform_(A, a=sqrt(5)) => U(-1/sqrt(fan_in), +1/sqrt(fan_in)); B = 0
-  const float bound = 1.0f / sqrtf(static_cast<float>(d));
   uint64_t x = seed ? seed : 0x9E3779B97F4A7C15ull;
   auto next = [&]() {
     x += 0x9E3779B97F4A7C15ull;
@@ -1585,8 +1726,10 @@ int32_t dtx_init_lora(dtx_trainer* t, uint64_t seed) {
   };
   for (int64_t l = 0; l < t->mc.n_layers; ++l)
     for (int ti = 0; ti < t->nt; ++ti) {
+      const int64_t d_in = t->tg[ti].d_in;
+      const float bound = 1.0f / sqrtf(static_cast<float>(d_in));
       float* a = host.data() + l * t->per_layer + t->tg[ti].off;
-      for (int64_t i = 0; i < d * r; ++i) a[i] = (2.f * next() - 1.f) * bound;
+      for (int64_t i = 0; i < d_in * r; ++i) a[i] = (2.f * next() - 1.f) * bound;
     }
   CKM(upload_sync(t->params, host.data(), host.size() * 4, t->stream));
   CKM(cudaMemsetAsync(t->adam_m, 0, t->n_train * 4, t->stream));
@@ -1792,31 +1935,27 @@ static int32_t export_lora_tensor(dtx_trainer* t, const float* flat, const char*
   if (!t || !name || !host_out) return t ? t->fail(DTX_ERR_INVALID, "null argument") : DTX_ERR_INVALID;
   if (t->full || !flat) return t->fail(DTX_ERR_STATE, "no adapters: this trainer was created for full-parameter SFT");
   cudaSetDevice(t->device);
-  const int64_t d = t->mc.hidden, r = t->tc.lora_r;
+  const int64_t r = t->tc.lora_r;
   int layer = -1;
   const char* rest = nullptr;
   if (!parse_layer(name, &layer, &rest) || layer < 0 || layer >= t->mc.n_layers)
     return t->fail(DTX_ERR_INVALID, "bad adapter tensor name %s", name);
-  char which = 0;
-  if (strstr(rest, "q_proj")) which = 'q';
-  else if (strstr(rest, "k_proj")) which = 'k';
-  else if (strstr(rest, "v_proj")) which = 'v';
-  const int ti = which ? target_index(t, which) : -1;
+  const int ti = target_index(t, rest);
   if (ti < 0) return t->fail(DTX_ERR_INVALID, "%s: module is not a LoRA target", name);
-  const int64_t d_out = t->tg[ti].d_out;
+  const int64_t d_in = t->tg[ti].d_in, d_out = t->tg[ti].d_out;
   const bool is_a = strstr(rest, "lora_A") != nullptr;
-  if (nbytes < (is_a ? d : d_out) * r * 4) return t->fail(DTX_ERR_INVALID, "%s: output buffer too small", name);
+  if (nbytes < (is_a ? d_in : d_out) * r * 4) return t->fail(DTX_ERR_INVALID, "%s: output buffer too small", name);
   const float* base = flat + static_cast<int64_t>(layer) * t->per_layer + t->tg[ti].off;
   CKM(cudaStreamSynchronize(t->stream));
-  std::vector<float> tmp(d * r);
+  std::vector<float> tmp(d_in * r);
   float* out = static_cast<float*>(host_out);
   if (strstr(rest, "lora_A")) {
-    CKM(cudaMemcpyAsync(tmp.data(), base, d * r * 4, cudaMemcpyDeviceToHost, t->stream));
+    CKM(cudaMemcpyAsync(tmp.data(), base, d_in * r * 4, cudaMemcpyDeviceToHost, t->stream));
     CKM(cudaStreamSynchronize(t->stream));
-    for (int64_t c = 0; c < d; ++c)
-      for (int64_t j = 0; j < r; ++j) out[j * d + c] = tmp[c * r + j];
+    for (int64_t c = 0; c < d_in; ++c)
+      for (int64_t j = 0; j < r; ++j) out[j * d_in + c] = tmp[c * r + j];
   } else if (strstr(rest, "lora_B")) {
-    CKM(cudaMemcpyAsync(out, base + d * r, d_out * r * 4, cudaMemcpyDeviceToHost, t->stream));
+    CKM(cudaMemcpyAsync(out, base + d_in * r, d_out * r * 4, cudaMemcpyDeviceToHost, t->stream));
     CKM(cudaStreamSynchronize(t->stream));
   } else {
     return t->fail(DTX_ERR_INVALID, "%s: expected lora_A or lora_B", name);

@@ -19,7 +19,9 @@ LIB_PATH = os.environ.get("DTX_LIB_PATH") or os.path.join(_HERE, "libdtxtune.so"
 
 DTX_F32, DTX_BF16, DTX_F16 = 0, 1, 2
 SCHED = {"linear": 0, "cosine": 1, "constant": 2, "constant_with_warmup": 3}
-TARGET_BITS = {"q_proj": 1, "k_proj": 2, "v_proj": 4}
+# LoRA target bits in HF module order (include/dtxtune.h); bit 8 (o_proj) is reserved: its adapter is not implemented
+TARGET_BITS = {"q_proj": 1, "k_proj": 2, "v_proj": 4, "gate_proj": 16, "up_proj": 32, "down_proj": 64}
+MLP_TARGETS = ("gate_proj", "up_proj", "down_proj")
 EPI_BF16, EPI_F32, EPI_BF16_ADD, EPI_ROPE, EPI_SWIGLU_FWD, EPI_SWIGLU_BWD = 0, 1, 2, 3, 4, 5
 STEP_FORCE = 1
 
@@ -53,7 +55,7 @@ ABI_SYMBOLS = [
     "dtx_base_weight_bytes", "dtx_last_step_ms", "dtx_last_step_timings", "dtx_last_step_groups", "dtx_plan_length_groups", "dtx_plan_packed_rows", "dtx_lr_lambda", "dtx_set_option", "dtx_gemm_bf16",
     "dtx_gemm_fused", "dtx_embedding_fwd", "dtx_rmsnorm_fwd", "dtx_rmsnorm_bwd",
     "dtx_rope_table", "dtx_rope_qk", "dtx_swiglu_fwd", "dtx_swiglu_bwd", "dtx_lora_dropout_fwd", "dtx_lora_dropout_bwd_add",
-    "dtx_nf4_roundtrip", "dtx_nf4_pack", "dtx_nf4_dequant", "dtx_cross_entropy", "dtx_sumsq", "dtx_adamw",
+    "dtx_swiglu_bwd_lora_dropout", "dtx_nf4_roundtrip", "dtx_nf4_pack", "dtx_nf4_dequant", "dtx_cross_entropy", "dtx_sumsq", "dtx_adamw",
     "dtx_attn_fwd", "dtx_attn_bwd",
 ]
 
@@ -120,6 +122,7 @@ def load() -> C.CDLL:
     lib.dtx_swiglu_bwd.argtypes = [vp, vp, vp, i32, i32, vp]
     lib.dtx_lora_dropout_fwd.argtypes = [vp, vp, i32, i32, i32, f32, C.c_uint64, vp]
     lib.dtx_lora_dropout_bwd_add.argtypes = [vp, vp, i32, i32, i32, f32, C.c_uint64, vp]
+    lib.dtx_swiglu_bwd_lora_dropout.argtypes = [vp, vp, vp, vp, i32, i32, i32, f32, C.c_uint64, vp]
     lib.dtx_cross_entropy.argtypes = [vp, i64, vp, vp, vp, vp, vp, i64, vp, i32, i32, i32, vp]
     lib.dtx_sumsq.argtypes = [vp, i64, vp, vp, vp]
     lib.dtx_adamw.argtypes = [vp, vp, vp, vp, i64, f32, f32, f32, f32, f32, i32, f32, vp, f32, vp, vp]
@@ -222,11 +225,25 @@ class TrainConfig:
         mask = 0
         for t in self.lora_target:
             if t not in TARGET_BITS:
-                raise DtxError(-5, f"lora_target {t!r} is not implemented natively (q_proj,k_proj,v_proj are)")
+                raise DtxError(-5, f"lora_target {t!r} is not implemented natively (q_proj,k_proj,v_proj,gate_proj,up_proj,down_proj "
+                                   "are; o_proj is the one linear module whose adapter is not)")
             mask |= TARGET_BITS[t]
         return TrainCfg(self.lora_r, self.lora_alpha, self.lora_dropout, mask, self.lr, self.weight_decay, self.beta1,
                         self.beta2, self.eps, self.max_grad_norm, SCHED[self.sched], self.warmup_steps, self.total_steps,
                         self.grad_accum, self.micro_batch, self.seq_len, self.seed, 1 if self.full_finetune else 0, 0)
+
+
+def module_path(target: str) -> str:
+    """Path of a LoRA target module inside a decoder layer: "mlp.gate_proj", "self_attn.q_proj"."""
+    return f"mlp.{target}" if target in MLP_TARGETS else f"self_attn.{target}"
+
+
+def linear_dims(model: ModelConfig, target: str) -> Tuple[int, int]:
+    """(in, out) features of a decoder layer's linear module."""
+    d, F = model.hidden, model.ffn
+    dkv = (model.n_kv_heads or model.n_heads) * model.head_dim
+    return {"q_proj": (d, d), "k_proj": (d, dkv), "v_proj": (d, dkv), "o_proj": (d, d), "gate_proj": (d, F), "up_proj": (d, F),
+            "down_proj": (F, d)}[target]
 
 
 _NP_DTYPES = {np.dtype(np.float32): DTX_F32, np.dtype(np.float16): DTX_F16}
@@ -342,19 +359,20 @@ class Trainer:
         for l in range(self.model.n_layers):
             for t in self.train.lora_target:
                 for ab in ("lora_A", "lora_B"):
-                    yield f"base_model.model.model.layers.{l}.self_attn.{t}.{ab}.weight"
+                    yield f"base_model.model.model.layers.{l}.{module_path(t)}.{ab}.weight"
+
+    def adapter_shape(self, name: str) -> Tuple[int, int]:
+        """peft's shape of an adapter tensor: lora_A [r, in], lora_B [out, r]."""
+        d_in, d_out = linear_dims(self.model, name.split(".lora_")[0].rsplit(".", 1)[-1])
+        return (self.train.lora_r, d_in) if "lora_A" in name else (d_out, self.train.lora_r)
 
     def export_adapter(self, grads: bool = False) -> Dict[str, np.ndarray]:
         """PEFT state dict (fp32): lora_A [r, in], lora_B [out, r] per target module.  grads=True returns, under the same
         names, the summed gradient the last optimizer step consumed."""
         out = {}
         fn = self.lib.dtx_export_adapter_grad if grads else self.lib.dtx_export_adapter
-        d, r = self.model.hidden, self.train.lora_r
-        dkv = (self.model.n_kv_heads or self.model.n_heads) * self.model.head_dim
         for name in self.adapter_names():
-            d_out = d if ".q_proj." in name else dkv
-            shape = (r, d) if "lora_A" in name else (d_out, r)
-            buf = np.empty(shape, dtype=np.float32)
+            buf = np.empty(self.adapter_shape(name), dtype=np.float32)
             check(fn(self._h, name.encode(), buf.ctypes.data_as(C.c_void_p), buf.nbytes), self._h)
             out[name] = buf
         return out

@@ -43,10 +43,23 @@ typedef enum { DTX_SCHED_LINEAR = 0, DTX_SCHED_COSINE = 1, DTX_SCHED_CONSTANT = 
                DTX_SCHED_CONSTANT_WITH_WARMUP = 3 } dtx_sched;
 
 /* LoRA target bits, in HF module order (cmd/tuning/parser.py:211-213 `--lora_target`; the controller
- * hard-codes "q_proj,v_proj": finetune_controller.go:482). */
+ * hard-codes "q_proj,v_proj": finetune_controller.go:482).  Any non-empty subset works.  Bit 8 (o_proj) is reserved: its
+ * adapter is not implemented and dtx_trainer_create refuses it with DTX_ERR_UNSUPPORTED.
+ *   bit   module                   lora_A [r, in]   lora_B [out, r]   input of the adapter
+ *   1     self_attn.q_proj         [r, hidden]      [hidden, r]       input_layernorm(x)
+ *   2     self_attn.k_proj         [r, hidden]      [kv_width, r]     input_layernorm(x)      (kv_width = n_kv_heads * head_dim)
+ *   4     self_attn.v_proj         [r, hidden]      [kv_width, r]     input_layernorm(x)
+ *   16    mlp.gate_proj            [r, hidden]      [ffn, r]          post_attention_layernorm(x)
+ *   32    mlp.up_proj              [r, hidden]      [ffn, r]          post_attention_layernorm(x)
+ *   64    mlp.down_proj            [r, ffn]         [hidden, r]       silu(gate) * up
+ * Tensor names are "model.layers.N.<module>.lora_A.weight" / "...lora_B.weight" (a "base_model.model." prefix is accepted).
+ * A is initialised U(-1/sqrt(in), 1/sqrt(in)), B = 0; one independent dropout mask per module. */
 #define DTX_TARGET_Q 1u
 #define DTX_TARGET_K 2u
 #define DTX_TARGET_V 4u
+#define DTX_TARGET_GATE 16u
+#define DTX_TARGET_UP 32u
+#define DTX_TARGET_DOWN 64u
 
 /* Architecture of the frozen base model: the fields of HF config.json that LlamaForCausalLM reads
  * (loaded by AutoConfig at cmd/tuning/train.py:221). */
@@ -151,6 +164,8 @@ DTX_API int32_t dtx_export_adapter_grad(dtx_trainer* t, const char* hf_name, voi
 /* Full-parameter SFT: one weight (grad = 0) or its accumulated gradient (grad = 1) by HF checkpoint name, as bf16 bit patterns
  * in the HF layout - what trainer.save_model writes for a full fine-tune. */
 DTX_API int32_t dtx_export_weight(dtx_trainer* t, const char* hf_name, void* host_out_bf16, int64_t nbytes, int32_t grad);
+/* trainable parameters: LoRA = n_layers * sum over the enabled targets of r * (in + out) (Llama-2-7B at r = 16: q,v 8 388 608;
+ * gate,up,down 23 199 744; q,k,v,gate,up,down 35 782 656); full-parameter SFT = every weight */
 DTX_API int64_t dtx_num_trainable(const dtx_trainer* t);
 /* kernels launched by this trainer since creation (bench.py's gpu_launches) */
 DTX_API int64_t dtx_launch_count(const dtx_trainer* t);
@@ -222,6 +237,12 @@ DTX_API int32_t dtx_swiglu_bwd(const void* dact, const void* gu, void* dgu, int3
 DTX_API int32_t dtx_lora_dropout_fwd(const void* h, void* hd, int32_t M, int32_t d, int32_t nt, float p, uint64_t key, void* stream);
 DTX_API int32_t dtx_lora_dropout_bwd_add(void* dh, const void* g, int32_t M, int32_t d, int32_t nt, float p, uint64_t key,
                                  void* stream);
+/* LoRA dropout on down_proj's input, backward, in one pass: dgu[M, 2F] = SwiGLU backward (as dtx_swiglu_bwd) of
+ * d(act) = dact + mask o g / (1 - p), where g [M, F] is the LoRA branch's input gradient and mask is the one
+ * dtx_lora_dropout_fwd(act, ., M, F, 1, p, key) drew.  interleaved = 0: gu / dgu rows are [gate F | up F]; 1: the
+ * GU-interleaved layout of the training step (feature f: gate at column (f/128)*256 + f%128, up 128 further). */
+DTX_API int32_t dtx_swiglu_bwd_lora_dropout(const void* dact, const void* g, const void* gu, void* dgu, int32_t M, int32_t F,
+                                            int32_t interleaved, float p, uint64_t key, void* stream);
 DTX_API int32_t dtx_nf4_roundtrip(void* w_bf16, int64_t n, void* stream);
 /* packed NF4 storage (bitsandbytes quantize_4bit layout: first element of a pair in the high nibble; one fp32 absmax per 64) */
 DTX_API int32_t dtx_nf4_pack(const void* w_bf16, void* packed_u8, void* absmax_f32, int64_t n, void* stream);
